@@ -1,8 +1,11 @@
 #!/usr/bin/env python
 """bench.py -- env-steps/s of the packing-environment hot path (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--config NAME]          # B200 arm, one JSON line on rank 0
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--config NAME] [--dump-outputs DIR]   # B200 arm, one JSON line on rank 0
     python bench.py --impl reference [--gpus N] --steps K --warmup W [--config NAME]   # reference CPU arm (oracle port)
+
+``--dump-outputs DIR`` writes what the last timed step returned to its caller (rank 0's bins) as ``DIR/<name>.npy``, so
+that two builds can be compared output for output: the inputs are seeded and identical from run to run.
 
 ``--config`` selects one of BASELINE.json's configurations (default ``blockout`` = configs[1], the one the
 metric is quoted on):
@@ -51,6 +54,7 @@ UNIT = "env-steps/s"
 CPU_ENVS_PER_CORE = 2    # bins per worker process of the CPU arm (same in cpu_baseline and --impl reference)
 CPU_SAMPLES = 3          # the CPU arm reports the median of this many timed samples
 DEFAULT_NCCL_CHANNELS = 0   # channels (= SMs) of the rollout all-gather; 0 = NCCL's default (see main_gpu)
+DUMP_LIMIT_BYTES = 64 * 10 ** 6   # --dump-outputs: larger outputs are written as a seeded sample of bins
 
 CONFIGS = {
     "blockout": dict(bins=4096, k=1, R=4, metric="env steps/sec (4096 bins, BlockOut)",
@@ -190,6 +194,30 @@ def device_policy(torch, obs, gen):
     mask = obs[:, :SEL * 5].view(n, SEL, 5)[:, :, 4] == 1
     score = torch.rand((n, SEL), device=obs.device, generator=gen) + mask.float()
     return torch.argmax(score, dim=1)
+
+
+def step_outputs(env, state):
+    """Host copies of what the last device-resident step handed its caller: the observation, the location candidates
+    it chose from (buffered) and the per-bin result arrays.  Integer and flag arrays become float64, which is exact."""
+    out = {"obs": state["obs"]}
+    if "loc" in state:
+        out["candidates"] = state["loc"]
+    out.update(env.last_step_device())
+    out = {k: v.cpu().numpy() for k, v in out.items()}
+    return {k: v if v.dtype in (np.float32, np.float64) else v.astype(np.float64) for k, v in out.items()}
+
+
+def dump_outputs(out_dir, arrays, limit=DUMP_LIMIT_BYTES, seed=0):
+    """Write every [N, ...] array of `arrays` as out_dir/<name>.npy and the bin index of each row as bins.npy.  When the
+    whole would exceed `limit` bytes, every array is cut to the same fixed, seeded sample of bins."""
+    n = len(arrays["obs"])
+    row_bytes = 8 + sum(a[:1].nbytes for a in arrays.values())
+    rows = min(n, (limit - 4096) // row_bytes)            # 4096: room for the .npy headers
+    bins = np.arange(n) if rows == n else np.sort(np.random.default_rng(seed).choice(n, rows, replace=False))
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "bins.npy"), bins.astype(np.float64))
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a[bins])
 
 
 def host_policy(rng, obs):
@@ -458,8 +486,8 @@ def main_gpu(args):
         if k > 1:
             if ev is not None:
                 ev[0].record()
-            loc = env.get_action_candidates(choice, as_tensor=True)
-            acts = device_policy(torch, loc, gen)       # the location agent needs the candidates: inside the interval
+            state["loc"] = env.get_action_candidates(choice, as_tensor=True)
+            acts = device_policy(torch, state["loc"], gen)   # the location agent needs the candidates: inside the interval
             state["obs"], _ = env.step_device(acts)
         else:
             if ev is not None:
@@ -532,6 +560,7 @@ def main_gpu(args):
     barrier()
     t_wall = time.perf_counter() - t_wall0
     launches_timed = env.launch_count() - launches0
+    outputs = step_outputs(env, state) if args.dump_outputs and rank == 0 else None   # before any further step
     # the timed region lasts ~10-30 ms: keep the same loop running (untimed) until nvidia-smi has
     # delivered enough clock samples under this load
     extra_steps = 0
@@ -674,6 +703,8 @@ def main_gpu(args):
             line["cpu_baseline"] = cpu_base
         print(json.dumps(line))
     env.close()
+    if outputs is not None:
+        dump_outputs(args.dump_outputs, outputs)
     if world > 1:
         dist.destroy_process_group()
     return 0
@@ -688,9 +719,12 @@ def main():
     ap.add_argument("--config", default="blockout", choices=sorted(CONFIGS))
     ap.add_argument("--cpu-seconds", type=float, default=15.0, help="bound of the cpu_baseline timed samples (wall seconds, all samples)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's outputs as DIR/<name>.npy")
     args = ap.parse_args()
     args.warmup = max(args.warmup, 3)
     if args.impl == "reference":
+        if args.dump_outputs:
+            raise SystemExit("--dump-outputs: only the B200 arm has a timed device step to dump")
         return main_reference(args)
     return main_gpu(args)
 

@@ -13,6 +13,7 @@ The GPU box has no reference tree; tests there read only the ``.npz`` files writ
 """
 import os
 import sys
+import zipfile
 
 import numpy as np
 
@@ -23,6 +24,15 @@ sys.path.insert(0, ROOT)
 from irbpp_b200 import shapes  # noqa: E402
 from oracle import ref_loader  # noqa: E402
 from oracle.oracle_env import HEURISTICS, OracleConfig, OracleVecEnv, RefGeometry  # noqa: E402
+
+
+def savez(path, **arrays):
+    """``np.savez_compressed`` at zlib's highest level: keeps every fixture under 1 MB (episode_irregular.npz is just
+    over at the default level).  ``np.load`` reads it like any .npz."""
+    with zipfile.ZipFile(path, "w", zipfile.ZIP_DEFLATED, compresslevel=9) as z:
+        for name, a in arrays.items():
+            with z.open(name + ".npy", "w", force_zip64=True) as f:
+                np.lib.format.write_array(f, np.asanyarray(a), allow_pickle=False)
 
 
 def lib_arrays(lib, prefix="lib_"):
@@ -227,7 +237,7 @@ def main():
     # (--buffered10-only) so the round-1 fixtures stay byte-identical.
     if "--buffered10-only" in sys.argv or "--all" in sys.argv:
         d = gen_episode("buffered10", shapes.make_blockout_library(16, seed=8), 4, 3, 36, 29, bufferSize=10)
-        np.savez_compressed(os.path.join(HERE, "episode_buffered10.npz"), **d)
+        savez(os.path.join(HERE, "episode_buffered10.npz"), **d)
         if "--buffered10-only" in sys.argv:
             return
     heur = {
@@ -235,13 +245,13 @@ def main():
         "heuristic_irregular": gen_heuristic_episode("heur-irregular", shapes.make_irregular_library(12, seed=7), 8, 3, 48, 27),
     }
     for k, d in heur.items():
-        np.savez_compressed(os.path.join(HERE, k + ".npz"), **d)
+        savez(os.path.join(HERE, k + ".npz"), **d)
     if "--heuristics-only" in sys.argv:
         return
     for tag, d in gen_scan_cases(space_mod).items():
-        np.savez_compressed(os.path.join(HERE, "scan_%s.npz" % tag), **d)
-    np.savez_compressed(os.path.join(HERE, "hulls.npz"), **gen_hull_cases(cv_mod))
-    np.savez_compressed(os.path.join(HERE, "kats.npz"), **gen_kats(cv_mod))
+        savez(os.path.join(HERE, "scan_%s.npz" % tag), **d)
+    savez(os.path.join(HERE, "hulls.npz"), **gen_hull_cases(cv_mod))
+    savez(os.path.join(HERE, "kats.npz"), **gen_kats(cv_mod))
     eps = {
         "episode_blockout": gen_episode("blockout", shapes.make_blockout_library(16, seed=1), 4, 4, 70, 21),
         "episode_irregular": gen_episode("irregular", shapes.make_irregular_library(16, seed=2), 8, 4, 50, 22),
@@ -255,7 +265,7 @@ def main():
         "episode_rot24": gen_episode("rot24", shapes.make_irregular_library(8, seed=9, num_rotations=24), 24, 2, 24, 28),
     }
     for k, d in eps.items():
-        np.savez_compressed(os.path.join(HERE, k + ".npz"), **d)
+        savez(os.path.join(HERE, k + ".npz"), **d)
     import cv2
     with open(os.path.join(HERE, "PROVENANCE.txt"), "w") as f:
         f.write("generated by tests/golden/make_golden.py from the unmodified reference at %s\n" % ref_loader.REFERENCE_ROOT)
