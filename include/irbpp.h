@@ -26,7 +26,7 @@
 extern "C" {
 #endif
 
-#define IRBPP_ABI_VERSION 1
+#define IRBPP_ABI_VERSION 2
 
 #define IRBPP_OK        0
 #define IRBPP_EINVAL   -1   /* bad argument / unsupported configuration */
@@ -219,6 +219,69 @@ int irbpp_shape_features(const float* shape_array, int32_t S, int32_t P, const f
                          int32_t item_col, const int32_t* ids, int32_t B, uint64_t seed, uint64_t counter,
                          int32_t n_points, const float* W1, const float* b1, const float* W2, const float* b2,
                          float negative_slope, int32_t* scratch_keys, float* out, void* stream);
+
+/* ---- prioritized n-step replay, one bank per bin (SURVEY.md 8(f)2; csrc/irbpp_replay.cuh) ------------------------
+ * Replaces: the N ReplayMemory objects of main.py:61-63 (memory.py:95-208), their appends in trainer.py:184-186 and the
+ * sample / update_priorities calls of agent.py:68-124.  Bank b is exactly ReplayMemory(args, capacity, obs_len): a
+ * sum tree of 2C-1 float32 nodes (leaves C-1 .. 2C-2, any C), a cyclic slot index, `full`, the running max priority
+ * (starts at 1) and the episode timestep t.  Handle-free: the caller owns every buffer (device pointers); the calls
+ * are ordered on `stream` and none synchronises with the host; errors through irbpp_last_error(NULL). */
+#define IRBPP_REPLAY_MAX_STEPS 16
+
+typedef struct irbpp_replay_banks {
+    int32_t  num_banks;        /* N */
+    int32_t  capacity;         /* C transitions per bank */
+    int32_t  obs_len;          /* L floats per state */
+    int32_t  row_stride;       /* floats between stored states: >= obs_len, a multiple of 4 (16-byte aligned rows) */
+    float*   tree;             /* [N, 2C-1] sum trees */
+    float*   states;           /* [N, C, row_stride] */
+    int64_t* actions;          /* [N, C] */
+    float*   rewards;          /* [N, C] */
+    uint8_t* nonterminals;     /* [N, C] */
+    int32_t* index;            /* [N] next slot (transitions.index) */
+    uint8_t* full;             /* [N] */
+    float*   max_priority;     /* [N] transitions.max, 1 initially */
+    int32_t* timestep;         /* [N] ReplayMemory.t */
+} irbpp_replay_banks;
+
+/* memory.py:110-113 for every bank b with valid[b] != 0 (valid may be NULL: all):  state row b (stride state_stride
+ * floats), action[b] (int64), reward[b] (float32, clamped to +-reward_clip when reward_clip > 0, trainer.py:181-182),
+ * done[b] (uint8).  Reads the step's arrays in stream order (e.g. irbpp_device_results), so it can follow a step in
+ * the same stream or CUDA graph without a host round trip. */
+int irbpp_replay_append(const irbpp_replay_banks* banks, const float* state, int64_t state_stride, const int64_t* action,
+                        const float* reward, const uint8_t* done, const uint8_t* valid, float reward_clip, void* stream);
+
+/* ReplayMemory.sample (memory.py:191-203) as agent.learn draws it (agent.py:68-82).  N <= batch: every bank gives
+ * batch / N stratified draws; N > batch: `batch` banks chosen uniformly without replacement on the device, one draw each
+ * (the reference's formula then gives every weight 1).  Rows = banks * per, bank-major.  Draw (row, attempt) uses
+ * u_table[row * max_attempts + attempt] (device float64) when u_table is not NULL, else a counter-based stream of
+ * (seed, counter); a row still rejected after max_attempts gets error[row] = 1 (the reference would retry forever).
+ * Outputs (device): banks int32 [rows / per], tree_index int64 [rows] = bank * (2C-1) + node, states / next_states
+ * float32 [rows, obs_len], actions int64 [rows], returns / nonterminals / weights float32 [rows], error int32 [rows]. */
+typedef struct irbpp_replay_sample_args {
+    int32_t       batch;
+    int32_t       multi_step;                             /* n <= IRBPP_REPLAY_MAX_STEPS */
+    float         n_step_scaling[IRBPP_REPLAY_MAX_STEPS]; /* float32(discount ** k), memory.py:107 */
+    double        priority_weight;                        /* beta */
+    uint64_t      seed, counter;
+    const double* u_table;
+    int32_t       max_attempts;
+    int32_t*      banks;
+    int64_t*      tree_index;
+    float*        states;
+    int64_t*      actions;
+    float*        returns;
+    float*        next_states;
+    float*        nonterminals;
+    float*        weights;
+    int32_t*      error;
+} irbpp_replay_sample_args;
+int irbpp_replay_sample(const irbpp_replay_banks* banks, const irbpp_replay_sample_args* args, void* stream);
+
+/* ReplayMemory.update_priorities after np.power (memory.py:206-208): tree_index int64 [count] as irbpp_replay_sample
+ * returned it, priority float32 [count] (device); applied in order (a later duplicate wins), max over every value. */
+int irbpp_replay_update_priorities(const irbpp_replay_banks* banks, const int64_t* tree_index, const float* priority,
+                                   int32_t count, void* stream);
 
 /* Profiling aid: when enabled, thread 0 of every CTA adds the SM cycles it spent in each kernel phase
  * (0 scan kernel: load + apply action, 1 scan kernel: observation heightmap + scan + level bitmaps,

@@ -12,7 +12,7 @@ c_i32, c_i64, c_f64 = ctypes.c_int32, ctypes.c_int64, ctypes.c_double
 c_void_p, c_char_p = ctypes.c_void_p, ctypes.c_char_p
 
 IRBPP_OK, IRBPP_EINVAL, IRBPP_ECUDA, IRBPP_ESTATE, IRBPP_EDEVICE = 0, -1, -2, -3, -4
-ABI_VERSION = 1
+ABI_VERSION = 2
 
 
 class IrbppConfig(ctypes.Structure):
@@ -24,6 +24,24 @@ class IrbppConfig(ctypes.Structure):
 class IrbppStepResult(ctypes.Structure):
     _fields_ = [("reward", c_void_p), ("done", c_void_p), ("valid", c_void_p), ("error", c_void_p),
                 ("counter", c_void_p), ("ep_len", c_void_p), ("ratio", c_void_p), ("ep_reward", c_void_p)]
+
+
+class IrbppReplayBanks(ctypes.Structure):
+    _fields_ = [("num_banks", c_i32), ("capacity", c_i32), ("obs_len", c_i32), ("row_stride", c_i32),
+                ("tree", c_void_p), ("states", c_void_p), ("actions", c_void_p), ("rewards", c_void_p),
+                ("nonterminals", c_void_p), ("index", c_void_p), ("full", c_void_p), ("max_priority", c_void_p),
+                ("timestep", c_void_p)]
+
+
+REPLAY_MAX_STEPS = 16
+
+
+class IrbppReplaySampleArgs(ctypes.Structure):
+    _fields_ = [("batch", c_i32), ("multi_step", c_i32), ("n_step_scaling", ctypes.c_float * REPLAY_MAX_STEPS),
+                ("priority_weight", c_f64), ("seed", ctypes.c_uint64), ("counter", ctypes.c_uint64),
+                ("u_table", c_void_p), ("max_attempts", c_i32), ("banks", c_void_p), ("tree_index", c_void_p),
+                ("states", c_void_p), ("actions", c_void_p), ("returns", c_void_p), ("next_states", c_void_p),
+                ("nonterminals", c_void_p), ("weights", c_void_p), ("error", c_void_p)]
 
 
 # symbol -> (restype, argtypes); every symbol of include/irbpp.h appears here (checked by the tests)
@@ -59,6 +77,10 @@ SIGNATURES = {
                                      ctypes.c_uint64, c_i32, c_void_p, c_void_p, c_void_p, c_void_p, ctypes.c_float,
                                      c_void_p, c_void_p, c_void_p]),
     "irbpp_debug_phase_cycles": (c_i32, [c_void_p, c_i32, c_void_p]),
+    "irbpp_replay_append": (c_i32, [ctypes.POINTER(IrbppReplayBanks), c_void_p, c_i64, c_void_p, c_void_p, c_void_p,
+                                    c_void_p, ctypes.c_float, c_void_p]),
+    "irbpp_replay_sample": (c_i32, [ctypes.POINTER(IrbppReplayBanks), ctypes.POINTER(IrbppReplaySampleArgs), c_void_p]),
+    "irbpp_replay_update_priorities": (c_i32, [ctypes.POINTER(IrbppReplayBanks), c_void_p, c_void_p, c_i32, c_void_p]),
 }
 
 _LIB = None

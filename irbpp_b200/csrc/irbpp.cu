@@ -19,6 +19,7 @@
 #include "irbpp_kernels.cuh"
 #include "irbpp_pointnet.cuh"
 #include "irbpp_pack.cuh"
+#include "irbpp_replay.cuh"
 
 using namespace irbpp;
 
@@ -857,6 +858,69 @@ int irbpp_shape_features(const float* shape_array, int32_t S, int32_t P, const f
     e = cudaGetLastError();
     if (e != cudaSuccess) return fail(nullptr, IRBPP_ECUDA, "kernel launch: %s", cudaGetErrorString(e));
     return IRBPP_OK;
+}
+
+// ---- prioritized n-step replay banks (SURVEY.md 8(f)2; csrc/irbpp_replay.cuh) ---------------------------------------
+static int replay_check(const irbpp_replay_banks* b) {
+    if (!b || b->num_banks <= 0 || b->capacity <= 0 || b->obs_len <= 0 || b->row_stride < b->obs_len || (b->row_stride & 3))
+        return fail(nullptr, IRBPP_EINVAL, "bad replay bank descriptor");
+    if (!b->tree || !b->states || !b->actions || !b->rewards || !b->nonterminals || !b->index || !b->full ||
+        !b->max_priority || !b->timestep || (reinterpret_cast<uintptr_t>(b->states) & 15))
+        return fail(nullptr, IRBPP_EINVAL, "replay bank: null or misaligned buffer");
+    return IRBPP_OK;
+}
+
+static int launch_status(const char* what) {
+    cudaError_t e = cudaGetLastError();
+    if (e != cudaSuccess) return fail(nullptr, IRBPP_ECUDA, "%s launch: %s", what, cudaGetErrorString(e));
+    return IRBPP_OK;
+}
+
+int irbpp_replay_append(const irbpp_replay_banks* banks, const float* state, int64_t state_stride, const int64_t* action,
+                        const float* reward, const uint8_t* done, const uint8_t* valid, float reward_clip, void* stream) {
+    int rc = replay_check(banks); if (rc) return rc;
+    if (!state || !action || !reward || !done || state_stride < banks->obs_len)
+        return fail(nullptr, IRBPP_EINVAL, "bad replay append arguments");
+    DeviceGuard guard(device_of(banks->tree));
+    irbpp_replay_append_kernel<<<banks->num_banks, REPLAY_APPEND_THREADS, 0, (cudaStream_t)stream>>>(
+        *banks, state, state_stride, action, reward, done, valid, reward_clip);
+    return launch_status("replay append");
+}
+
+int irbpp_replay_sample(const irbpp_replay_banks* banks, const irbpp_replay_sample_args* a, void* stream) {
+    int rc = replay_check(banks); if (rc) return rc;
+    if (!a || a->batch <= 0 || a->multi_step < 0 || a->multi_step > IRBPP_REPLAY_MAX_STEPS || a->max_attempts <= 0 ||
+        !a->banks || !a->tree_index || !a->states || !a->actions || !a->returns || !a->next_states || !a->nonterminals ||
+        !a->weights || !a->error)
+        return fail(nullptr, IRBPP_EINVAL, "bad replay sample arguments");
+    const int N = banks->num_banks;
+    const bool choose = N > a->batch;                       // agent.py:69 would give 0 draws per memory
+    const int m = choose ? a->batch : N, per = choose ? 1 : a->batch / N;
+    ReplaySampleParams S;
+    memset(&S, 0, sizeof(S));
+    S.per = per; S.n = a->multi_step;
+    for (int k = 0; k < a->multi_step; ++k) S.scale[k] = a->n_step_scaling[k];
+    S.neg_beta = (float)(-a->priority_weight); S.beta_is_one = a->priority_weight == 1.0;
+    S.seed = a->seed; S.counter = a->counter; S.u_table = a->u_table; S.max_attempts = a->max_attempts;
+    S.banks = a->banks; S.choose = choose;
+    S.tree_index = a->tree_index; S.states = a->states; S.actions = a->actions; S.returns = a->returns;
+    S.next_states = a->next_states; S.nonterminals = a->nonterminals; S.weights = a->weights; S.error = a->error;
+    DeviceGuard guard(device_of(banks->tree));
+    cudaStream_t s = (cudaStream_t)stream;
+    if (choose) irbpp_replay_choose_kernel<<<1, 32, 0, s>>>(a->banks, m, N, a->seed, a->counter);
+    const int warps = std::min(per, REPLAY_MAX_WARPS);
+    irbpp_replay_sample_kernel<<<m, warps * 32, 0, s>>>(*banks, S);
+    return launch_status("replay sample");
+}
+
+int irbpp_replay_update_priorities(const irbpp_replay_banks* banks, const int64_t* tree_index, const float* priority,
+                                   int32_t count, void* stream) {
+    int rc = replay_check(banks); if (rc) return rc;
+    if (count < 0 || (count > 0 && (!tree_index || !priority))) return fail(nullptr, IRBPP_EINVAL, "bad replay update arguments");
+    if (count == 0) return IRBPP_OK;
+    DeviceGuard guard(device_of(banks->tree));
+    irbpp_replay_update_kernel<<<1, REPLAY_UPDATE_THREADS, 0, (cudaStream_t)stream>>>(*banks, tree_index, priority, count);
+    return launch_status("replay update");
 }
 
 int irbpp_debug_phase_cycles(irbpp_handle h, int32_t enable, uint64_t* out8) {

@@ -15,9 +15,9 @@ iteration rate.  This module keeps the loop's shape and removes the per-environm
   with the reference's segment rule made safe for N > batch_size (``segment_size``);
 * ``segment_size``         -- the shim for ``agent.py:69``.
 
-The replay bank samples uniformly (n-step returns and priorities live in the learner's ``memory.py``, which is out
-of this path's scope); it exists so that the actor loop can be run end to end at N = 4096 and timed
-(``tools/actor_loop.py``).
+``ReplayBank`` samples uniformly, without priorities or n-step returns; it exists so that the actor loop can be run end
+to end at N = 4096 and timed (``tools/actor_loop.py``).  The reference's learner memory (prioritized n-step replay,
+``memory.py``) at N = 4096 is ``irbpp_b200.replay.PrioritizedReplayBank``, which also uses ``segment_size``.
 """
 from collections import deque
 
