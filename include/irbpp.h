@@ -51,10 +51,12 @@ typedef struct irbpp_config {
     int32_t approx_legacy;     /* 0: approxPolyDP as cv2 4.13 (segment distance); 1: legacy line distance */
 } irbpp_config;
 
-/* Host views of the per-env results of the last step (library-owned pinned memory; two blocks alternate, so the
- * views stay valid until the SECOND next irbpp_step_async on the handle).  Replaces the (rews, dones, infos) tuple of
- * ShmemVecEnv.step_wait (wrapper/shmem_vec_env.py:76-81) and the Monitor episode info
- * (wrapper/monitor.py:58-75). */
+/* Views of the per-env results of the last step.  Replaces the (rews, dones, infos) tuple of ShmemVecEnv.step_wait
+ * (wrapper/shmem_vec_env.py:76-81) and the Monitor episode info (wrapper/monitor.py:58-75).  The eight arrays lie in
+ * one library-owned block of 31 bytes per env, in the order ratio | ep_reward | reward | counter | ep_len | done |
+ * valid | error.  irbpp_step_wait returns host views into one of two pinned blocks that alternate, so they stay valid
+ * until the SECOND next irbpp_step_async on the handle; irbpp_step_wait_device and irbpp_device_results return
+ * device views of the one device block (irbpp_device_result is the same struct). */
 typedef struct irbpp_step_result {
     const float*   reward;      /* [N]  10*volume/bin_volume on success, 0 otherwise (binPhy.py:299-322) */
     const uint8_t* done;        /* [N]  1 when the placement failed and the bin was auto-reset */
@@ -67,16 +69,7 @@ typedef struct irbpp_step_result {
 } irbpp_step_result;
 
 /* Device-resident copies of the same arrays (for callers that keep the loop on the GPU). */
-typedef struct irbpp_device_result {
-    const float*   reward;
-    const uint8_t* done;
-    const uint8_t* valid;
-    const uint8_t* error;
-    const int32_t* counter;
-    const int32_t* ep_len;
-    const double*  ratio;
-    const double*  ep_reward;
-} irbpp_device_result;
+typedef irbpp_step_result irbpp_device_result;
 
 int irbpp_abi_version(void);
 
@@ -167,8 +160,8 @@ int irbpp_step_poses_async(irbpp_handle h, const int64_t* poses, int32_t poses_o
 
 /* ---- parity / debugging views (float64, host destinations; any pointer may be NULL) ---- */
 
-/* Current bin state: heightmap [N,Hx,Hy] row-major, the candidate table [N,selected_action,5]
- * (rot, x, y decoded from the packed state; H and V columns are 0), next item ids [N, max(k,1)]. */
+/* Current bin state: heightmap [N,Hx,Hy] row-major; int32 next item ids queue [N, max(k,1)], sequence
+ * cursor [N] and packed_count [N], the items packed in the current episode. */
 int irbpp_debug_state(irbpp_handle h, double* heightmap, int32_t* queue, int32_t* cursor,
                       int32_t* packed_count);
 int irbpp_debug_set_heightmap(irbpp_handle h, const double* heightmap /* host [N,Hx,Hy] */);

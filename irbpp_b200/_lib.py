@@ -5,6 +5,8 @@ device is present ``irbpp_create`` fails with ``IRBPP_ECUDA``."""
 import ctypes
 import os
 
+import numpy as np
+
 HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("IRBPP_LIB") or os.path.join(HERE, "lib", "libirbpp.so")   # IRBPP_LIB: build-variant experiments
 
@@ -24,6 +26,22 @@ class IrbppConfig(ctypes.Structure):
 class IrbppStepResult(ctypes.Structure):
     _fields_ = [("reward", c_void_p), ("done", c_void_p), ("valid", c_void_p), ("error", c_void_p),
                 ("counter", c_void_p), ("ep_len", c_void_p), ("ratio", c_void_p), ("ep_reward", c_void_p)]
+
+
+# The block the pointers of IrbppStepResult point into: one array of N per field, in this order
+# (csrc/irbpp_kernels.cuh carve_results states the same layout).
+RESULT_FIELDS = (("ratio", np.dtype(np.float64)), ("ep_reward", np.dtype(np.float64)), ("reward", np.dtype(np.float32)),
+                 ("counter", np.dtype(np.int32)), ("ep_len", np.dtype(np.int32)), ("done", np.dtype(np.uint8)),
+                 ("valid", np.dtype(np.uint8)), ("error", np.dtype(np.uint8)))
+
+
+def result_offsets(n):
+    """Byte offset of every array in the result block of n bins, and the size of the block."""
+    offsets, size = {}, 0
+    for name, dt in RESULT_FIELDS:
+        offsets[name] = size
+        size += n * dt.itemsize
+    return offsets, size
 
 
 class IrbppReplayBanks(ctypes.Structure):

@@ -41,16 +41,14 @@ struct irbpp_env {
     int64_t launches = 0;
     // device allocations
     std::vector<void*> dev_allocs;
-    void* results_dev = nullptr;   // one block: ratio | ep_reward | reward | counter | ep_len | done | valid | error
-    void* results_host = nullptr;  // pinned mirror of the CURRENT step (one of results_host2[]: the blocks alternate, so the
-                                   // views of step k stay valid until step k + 2 is launched)
-    void* results_host2[2] = {nullptr, nullptr};
-    char* results_mapped2[2] = {nullptr, nullptr};
+    void* results_dev = nullptr;            // the device result block (carve_results)
+    void* results_host[2] = {nullptr, nullptr};   // pinned mirrors; the current step's is results_host[res_turn]: the blocks
+                                                  // alternate, so the views of step k stay valid until step k + 2 is launched
+    StepResults results_mapped[2] = {};     // device views of results_host[]
     int res_turn = 0;
     size_t results_bytes = 0;
     int64_t* actions_dev = nullptr;
     int64_t* actions_pinned = nullptr;      // [2][N] pinned staging: step actions, order actions
-    char* results_mapped = nullptr;         // device view of results_host
     uint8_t* which_dev = nullptr;
     // shape pools
     ShapeRot* srot_dev = nullptr; double* Bs_dev = nullptr; double* Ts_dev = nullptr;
@@ -219,28 +217,18 @@ int irbpp_create(const irbpp_config* cfg, irbpp_handle* out) {
     TRY_ALLOC(dev_alloc(h, &P.nlevels, units * P.R));
     if (!lists_in_smem(P.R)) TRY_ALLOC(dev_alloc(h, &P.dlist, units * 2 * P.R * NPOSE));
     TRY_ALLOC(dev_alloc(h, &h->ready_dev, units));        // zeroed: no launch has epoch 0
-    // result block (8-byte fields first so every array stays aligned)
-    h->results_bytes = (size_t)N * (8 + 8 + 4 + 4 + 4 + 1 + 1 + 1);
+    h->results_bytes = (size_t)N * RESULT_BYTES_PER_BIN;
     TRY_ALLOC(cudaMalloc(&h->results_dev, h->results_bytes + 64));
     TRY_ALLOC(cudaMemset(h->results_dev, 0, h->results_bytes + 64));
+    P.res = carve_results(h->results_dev, N);
     for (int t = 0; t < 2; ++t) {
-        TRY_ALLOC(cudaHostAlloc(&h->results_host2[t], h->results_bytes + 64, cudaHostAllocMapped));
-        TRY_ALLOC(cudaHostGetDevicePointer((void**)&h->results_mapped2[t], h->results_host2[t], 0));
-        memset(h->results_host2[t], 0, h->results_bytes + 64);
+        void* mapped = nullptr;
+        TRY_ALLOC(cudaHostAlloc(&h->results_host[t], h->results_bytes + 64, cudaHostAllocMapped));
+        TRY_ALLOC(cudaHostGetDevicePointer(&mapped, h->results_host[t], 0));
+        memset(h->results_host[t], 0, h->results_bytes + 64);
+        h->results_mapped[t] = carve_results(mapped, N);
     }
-    h->results_host = h->results_host2[0]; h->results_mapped = h->results_mapped2[0];
     TRY_ALLOC(cudaHostAlloc((void**)&h->actions_pinned, 2 * (size_t)N * sizeof(int64_t), cudaHostAllocMapped));
-    {
-        char* b = reinterpret_cast<char*>(h->results_dev);
-        P.r_ratio = reinterpret_cast<double*>(b); b += (size_t)N * 8;
-        P.r_eprew = reinterpret_cast<double*>(b); b += (size_t)N * 8;
-        P.r_reward = reinterpret_cast<float*>(b); b += (size_t)N * 4;
-        P.r_counter = reinterpret_cast<int32_t*>(b); b += (size_t)N * 4;
-        P.r_eplen = reinterpret_cast<int32_t*>(b); b += (size_t)N * 4;
-        P.r_done = reinterpret_cast<uint8_t*>(b); b += N;
-        P.r_valid = reinterpret_cast<uint8_t*>(b); b += N;
-        P.r_error = reinterpret_cast<uint8_t*>(b);
-    }
     TRY_ALLOC(raise_dynamic_smem(cfg->device, h->epc == ENVS_PER_CTA_WIDE ? 3 : 0, h->cand_smem));
 #undef TRY_ALLOC
     *out = h;
@@ -253,7 +241,7 @@ int irbpp_destroy(irbpp_handle h) {
     cudaDeviceSynchronize();
     for (void* p : h->dev_allocs) cudaFree(p);
     if (h->results_dev) cudaFree(h->results_dev);
-    for (int t = 0; t < 2; ++t) if (h->results_host2[t]) cudaFreeHost(h->results_host2[t]);
+    for (int t = 0; t < 2; ++t) if (h->results_host[t]) cudaFreeHost(h->results_host[t]);
     if (h->actions_pinned) cudaFreeHost(h->actions_pinned);
     delete h;
     return IRBPP_OK;
@@ -366,7 +354,7 @@ int irbpp_load_shapes(irbpp_handle h, int32_t S, int32_t R, const int32_t* dims,
                     for (int j = 0; j < q.h; ++j) {
                         const double b = Bq[(size_t)i * q.h + j];
                         if (std::isinf(b)) continue;
-                        TileEntry e; e.off = 8 * (((j & 1) * HX + i) * (HY / 2) + (j >> 1)); e.pad = 0; e.b = b;
+                        TileEntry e; e.off = 8 * hm_index(i, j); e.pad = 0; e.b = b;
                         tiles.push_back(e);
                     }
                 q.ntiles = (int32_t)tiles.size() - q.tile_off;
@@ -533,17 +521,7 @@ static int step_async_impl(irbpp_env* h, const int64_t* actions, int32_t on_devi
         memcpy(h->actions_pinned, actions, (size_t)P.N * sizeof(int64_t));
         P.actions = h->actions_dev;
         h->res_turn ^= 1;                                   // this step's host block (the previous step's stays readable)
-        h->results_host = h->results_host2[h->res_turn]; h->results_mapped = h->results_mapped2[h->res_turn];
-        char* b = h->results_mapped;
-        const size_t N = P.N;
-        P.h_ratio = reinterpret_cast<double*>(b); b += N * 8;
-        P.h_eprew = reinterpret_cast<double*>(b); b += N * 8;
-        P.h_reward = reinterpret_cast<float*>(b); b += N * 4;
-        P.h_counter = reinterpret_cast<int32_t*>(b); b += N * 4;
-        P.h_eplen = reinterpret_cast<int32_t*>(b); b += N * 4;
-        P.h_done = reinterpret_cast<uint8_t*>(b); b += N;
-        P.h_valid = reinterpret_cast<uint8_t*>(b); b += N;
-        P.h_error = reinterpret_cast<uint8_t*>(b);
+        P.res_host = h->results_mapped[h->res_turn];
         // (One CUDA graph per step -- H2D copy + both kernels, instantiated per observation buffer -- was measured:
         // submit 12.8 -> 8.8 us, but the step's wait grew by as much, e2e 0.162 vs 0.155 ms; dropped.)
         CUDA_TRY(h, cudaMemcpyAsync(h->actions_dev, h->actions_pinned, (size_t)P.N * sizeof(int64_t), cudaMemcpyHostToDevice, s));
@@ -561,16 +539,9 @@ int irbpp_step_poses_async(irbpp_handle h, const int64_t* poses, int32_t on_devi
     return step_async_impl(h, poses, on_device, obs_out, stream, 1);
 }
 
-static void host_views(irbpp_env* h, char* b, irbpp_step_result* out) {
-    const size_t N = h->P.N;
-    out->ratio = reinterpret_cast<double*>(b); b += N * 8;
-    out->ep_reward = reinterpret_cast<double*>(b); b += N * 8;
-    out->reward = reinterpret_cast<float*>(b); b += N * 4;
-    out->counter = reinterpret_cast<int32_t*>(b); b += N * 4;
-    out->ep_len = reinterpret_cast<int32_t*>(b); b += N * 4;
-    out->done = reinterpret_cast<uint8_t*>(b); b += N;
-    out->valid = reinterpret_cast<uint8_t*>(b); b += N;
-    out->error = reinterpret_cast<uint8_t*>(b);
+static void export_results(const StepResults& r, irbpp_step_result* out) {
+    out->reward = r.reward; out->done = r.done; out->valid = r.valid; out->error = r.error;
+    out->counter = r.counter; out->ep_len = r.ep_len; out->ratio = r.ratio; out->ep_reward = r.ep_reward;
 }
 
 int irbpp_step_wait(irbpp_handle h, irbpp_step_result* out) {
@@ -579,11 +550,12 @@ int irbpp_step_wait(irbpp_handle h, irbpp_step_result* out) {
     if (!h->waiting_step) return fail(h, IRBPP_ESTATE, "not running an async step");   // vec_env.py:18-26
     cudaStream_t s = h->pending_stream;
     h->waiting_step = false;
+    void* block = h->results_host[h->res_turn];
     if (out && !h->results_on_host)            // a device-resident step waited for with the host call: fetch the block
-        CUDA_TRY(h, cudaMemcpyAsync(h->results_host, h->results_dev, h->results_bytes, cudaMemcpyDeviceToHost, s));
+        CUDA_TRY(h, cudaMemcpyAsync(block, h->results_dev, h->results_bytes, cudaMemcpyDeviceToHost, s));
     CUDA_TRY(h, cudaStreamSynchronize(s));
     if (out) {
-        host_views(h, reinterpret_cast<char*>(h->results_host), out);
+        export_results(carve_results(block, h->P.N), out);
         for (int i = 0; i < h->P.N; ++i)
             if (out->error[i]) return fail(h, IRBPP_EDEVICE, "env %d reported device error code %d", i, (int)out->error[i]);
     }
@@ -595,19 +567,13 @@ int irbpp_step_wait_device(irbpp_handle h, irbpp_device_result* out) {
     DeviceGuard guard(h->cfg.device);
     if (!h->waiting_step) return fail(h, IRBPP_ESTATE, "not running an async step");
     h->waiting_step = false;
-    if (out) {
-        out->ratio = h->P.r_ratio; out->ep_reward = h->P.r_eprew; out->reward = h->P.r_reward;
-        out->counter = h->P.r_counter; out->ep_len = h->P.r_eplen; out->done = h->P.r_done;
-        out->valid = h->P.r_valid; out->error = h->P.r_error;
-    }
+    if (out) export_results(h->P.res, out);
     return IRBPP_OK;
 }
 
 int irbpp_device_results(irbpp_handle h, irbpp_device_result* out) {
     if (!h || !out) return IRBPP_EINVAL;
-    out->ratio = h->P.r_ratio; out->ep_reward = h->P.r_eprew; out->reward = h->P.r_reward;
-    out->counter = h->P.r_counter; out->ep_len = h->P.r_eplen; out->done = h->P.r_done;
-    out->valid = h->P.r_valid; out->error = h->P.r_error;
+    export_results(h->P.res, out);
     return IRBPP_OK;
 }
 
@@ -687,8 +653,7 @@ int irbpp_debug_state(irbpp_handle h, double* heightmap, int32_t* queue, int32_t
         for (int e = 0; e < N; ++e)
             for (int x = 0; x < HX; ++x)
                 for (int y = 0; y < HY; ++y)
-                    heightmap[((size_t)e * HX + x) * HY + y] =
-                        raw[(size_t)e * HX * HY + ((y & 1) * HX + x) * (HY / 2) + (y >> 1)];
+                    heightmap[((size_t)e * HX + x) * HY + y] = raw[(size_t)e * HX * HY + hm_index(x, y)];
     }
     if (queue || cursor || packed_count) {
         std::vector<EnvState> st((size_t)N);
@@ -712,7 +677,7 @@ int irbpp_debug_set_heightmap(irbpp_handle h, const double* heightmap) {
     for (int e = 0; e < N; ++e)
         for (int x = 0; x < HX; ++x)
             for (int y = 0; y < HY; ++y)
-                raw[(size_t)e * HX * HY + ((y & 1) * HX + x) * (HY / 2) + (y >> 1)] = heightmap[((size_t)e * HX + x) * HY + y];
+                raw[(size_t)e * HX * HY + hm_index(x, y)] = heightmap[((size_t)e * HX + x) * HY + y];
     CUDA_TRY(h, cudaDeviceSynchronize());
     CUDA_TRY(h, cudaMemcpy(h->P.hm, raw.data(), raw.size() * 8, cudaMemcpyHostToDevice));
     return IRBPP_OK;
@@ -745,7 +710,7 @@ static int debug_run(irbpp_env* h, Params& P, double* posZmap, double* posZValid
     if (cand) DBG_TRY(cudaMemcpy(cand, d_cd, nc * 8, cudaMemcpyDeviceToHost));
     if (num_hull) DBG_TRY(cudaMemcpy(num_hull, d_nh, N * 4, cudaMemcpyDeviceToHost));
     std::vector<uint8_t> errs(N);
-    DBG_TRY(cudaMemcpy(errs.data(), P.r_error, N, cudaMemcpyDeviceToHost));
+    DBG_TRY(cudaMemcpy(errs.data(), P.res.error, N, cudaMemcpyDeviceToHost));
     cleanup();
 #undef DBG_TRY
     for (size_t i = 0; i < N; ++i) if (errs[i]) return fail(h, IRBPP_EDEVICE, "env %zu reported device error code %d", i, (int)errs[i]);

@@ -127,6 +127,29 @@ struct EnvState {
 };
 static_assert(sizeof(EnvState) == 128, "EnvState must be 128 bytes");
 
+// The per-bin results of a step, one array of N per field, in the field order of irbpp_step_result.
+struct StepResults {
+    float* reward; uint8_t* done; uint8_t* valid; uint8_t* error;
+    int32_t* counter; int32_t* ep_len; double* ratio; double* ep_reward;
+};
+
+// The arrays of N bins in one block: ratio | ep_reward | reward | counter | ep_len | done | valid | error, 8-byte fields
+// first so that every array stays aligned.  irbpp_b200/_lib.py RESULT_FIELDS states the same layout.
+constexpr size_t RESULT_BYTES_PER_BIN = 8 + 8 + 4 + 4 + 4 + 1 + 1 + 1;
+inline StepResults carve_results(void* block, size_t n) {
+    char* b = static_cast<char*>(block);
+    StepResults r;
+    r.ratio = reinterpret_cast<double*>(b);     b += n * 8;
+    r.ep_reward = reinterpret_cast<double*>(b); b += n * 8;
+    r.reward = reinterpret_cast<float*>(b);     b += n * 4;
+    r.counter = reinterpret_cast<int32_t*>(b);  b += n * 4;
+    r.ep_len = reinterpret_cast<int32_t*>(b);   b += n * 4;
+    r.done = reinterpret_cast<uint8_t*>(b);     b += n;
+    r.valid = reinterpret_cast<uint8_t*>(b);    b += n;
+    r.error = reinterpret_cast<uint8_t*>(b);
+    return r;
+}
+
 struct Params {
     // configuration
     int32_t N, R, sel, K;                // K = buffer_size (1 = online)
@@ -170,17 +193,31 @@ struct Params {
     int32_t env_lo, env_hi;              // bins [env_lo, env_hi) handled by this launch (the full range [0, N))
     // outputs
     float* obs;                          // [N][obs_stride] (+ slot offset in MODE_ALL_OBS)
-    float* r_reward; uint8_t* r_done; uint8_t* r_valid; uint8_t* r_error;
-    int32_t* r_counter; int32_t* r_eplen; double* r_ratio; double* r_eprew;
+    StepResults res;                     // the device result block
     double* dbg_cand; int32_t* dbg_nhull;
-    // host-mapped mirror of the result arrays (zero-copy stores; NULL on the device-resident path)
-    float* h_reward; uint8_t* h_done; uint8_t* h_valid; uint8_t* h_error;
-    int32_t* h_counter; int32_t* h_eplen; double* h_ratio; double* h_eprew;
+    StepResults res_host;                // host-mapped mirror of this step's results (zero-copy stores; NULL on the device-resident path)
     unsigned long long* phase_cycles;    // [8] summed SM cycles per phase (thread 0 of every CTA), or NULL
     int32_t mode;
 };
 
-__device__ __forceinline__ int hm_index(int x, int y) { return ((y & 1) * HX + x) * (HY / 2) + (y >> 1); }
+// A bin's step result, stored to the device block and to the host mirror when there is one.
+__device__ __forceinline__ void store_result(const Params& P, int env, float reward, uint8_t done, uint8_t valid,
+                                             int32_t counter, int32_t ep_len, double ratio, double ep_reward) {
+    auto put = [&](const StepResults& r) {
+        r.reward[env] = reward; r.done[env] = done; r.valid[env] = valid;
+        r.counter[env] = counter; r.ep_len[env] = ep_len; r.ratio[env] = ratio; r.ep_reward[env] = ep_reward;
+    };
+    put(P.res);
+    if (P.res_host.reward) put(P.res_host);
+}
+
+__device__ __forceinline__ void store_error(const Params& P, int env, uint8_t code) {
+    P.res.error[env] = code;
+    if (P.res_host.error) P.res_host.error[env] = code;
+}
+
+// Cell (x, y) of a bin's heightmap: plane y & 1 holds the columns of that parity.
+__host__ __device__ __forceinline__ int hm_index(int x, int y) { return ((y & 1) * HX + x) * (HY / 2) + (y >> 1); }
 
 // Counter-based item generator (stand-in for RandomItemCreator, IRcreator.py:26-33, when no explicit sequences
 // are loaded): id = mix(seed, env, draw counter) mod S -- i.i.d. uniform ids, no period, no memory.
@@ -611,12 +648,7 @@ __global__ void __launch_bounds__(CTA_THREADS, IRBPP_SCAN_MIN_CTAS) irbpp_scan_k
             const int nfill = P.K > 1 ? P.K : 1;
             if (ok) {
                 const double rew = rew_pf;
-                P.r_reward[env] = (float)rew; P.r_done[env] = 0; P.r_valid[env] = 1;
-                P.r_counter[env] = -1; P.r_eplen[env] = 0; P.r_ratio[env] = -1.0; P.r_eprew[env] = 0.0;
-                if (P.h_reward) {
-                    P.h_reward[env] = (float)rew; P.h_done[env] = 0; P.h_valid[env] = 1;
-                    P.h_counter[env] = -1; P.h_eplen[env] = 0; P.h_ratio[env] = -1.0; P.h_eprew[env] = 0.0;
-                }
+                store_result(P, env, (float)rew, 0, 1, -1, 0, -1.0, 0.0);
                 st_s.packed += 1; st_s.ep_len += 1;
                 st_s.vol_sum += vol_pf;
                 st_s.ep_rew += rew;
@@ -625,16 +657,7 @@ __global__ void __launch_bounds__(CTA_THREADS, IRBPP_SCAN_MIN_CTAS) irbpp_scan_k
                 for (int q = oa; q + 1 < nfill; ++q) queue_g[q] = queue_g[q + 1];
                 queue_g[nfill - 1] = draw();
             } else {
-                P.r_reward[env] = 0.0f; P.r_done[env] = 1; P.r_valid[env] = 1;
-                P.r_counter[env] = st_s.packed;
-                P.r_ratio[env] = st_s.vol_sum / P.binvol;
-                P.r_eplen[env] = st_s.ep_len + 1;
-                P.r_eprew[env] = st_s.ep_rew + 0.0;
-                if (P.h_reward) {
-                    P.h_reward[env] = 0.0f; P.h_done[env] = 1; P.h_valid[env] = 1;
-                    P.h_counter[env] = st_s.packed; P.h_ratio[env] = st_s.vol_sum / P.binvol;
-                    P.h_eplen[env] = st_s.ep_len + 1; P.h_eprew[env] = st_s.ep_rew + 0.0;
-                }
+                store_result(P, env, 0.0f, 1, 1, st_s.packed, st_s.ep_len + 1, st_s.vol_sum / P.binvol, st_s.ep_rew + 0.0);
                 st_s.packed = 0; st_s.ep_len = 0; st_s.vol_sum = 0.0; st_s.ep_rew = 0.0;
                 st_s.order_act = 0;
                 for (int q = 0; q < nfill; ++q) queue_g[q] = draw();   // reset(): clear + preview
@@ -675,7 +698,7 @@ __global__ void __launch_bounds__(CTA_THREADS, IRBPP_SCAN_MIN_CTAS) irbpp_scan_k
     if (!emit_loc) {
         // order observation: [next k item ids | heightmap]  (binPhy.py:229-230)
         for (int i = tid; i < P.K; i += CTA_THREADS) obs_g[i] = (float)queue_g[i];
-        if (tid == 0) { P.r_error[env] = (uint8_t)err_sh; if (P.h_error) P.h_error[env] = (uint8_t)err_sh; st_s.next_seq = next_seq; }
+        if (tid == 0) { store_error(P, env, (uint8_t)err_sh); st_s.next_seq = next_seq; }
         if (st_dirty && warp == 0) {
             __syncwarp();
             reinterpret_cast<uint32_t*>(P.state + env)[lane] = reinterpret_cast<const uint32_t*>(&st_s)[lane];
@@ -724,10 +747,8 @@ __global__ void __launch_bounds__(CTA_THREADS, IRBPP_SCAN_MIN_CTAS) irbpp_scan_k
     }
     __syncthreads();
     if (tid == 0) {
-        if (mode != MODE_ALL_OBS || err_sh) {      // (several CTAs per bin in MODE_ALL_OBS: only error codes are written)
-            P.r_error[env] = (uint8_t)err_sh;      // the candidates kernel may overwrite with its own code
-            if (P.h_error) P.h_error[env] = (uint8_t)err_sh;
-        }
+        // (several CTAs per bin in MODE_ALL_OBS: only error codes are written; the candidates kernel may overwrite with its own code)
+        if (mode != MODE_ALL_OBS || err_sh) store_error(P, env, (uint8_t)err_sh);
         const bool write_state = (mode == MODE_STEP || mode == MODE_RESET || mode == MODE_CANDIDATES ||
                                   (mode == MODE_ALL_OBS && slot == P.K - 1));
         if (write_state) { st_s.cur_item = item; st_s.mask_any = any_sh; }
@@ -779,7 +800,7 @@ __global__ void __launch_bounds__(CTA_THREADS) irbpp_levels_kernel(const Params 
     }
     if (err) err_sh = 4;
     __syncthreads();
-    if (threadIdx.x == 0) P.r_error[env] = (uint8_t)err_sh;
+    if (threadIdx.x == 0) store_error(P, env, (uint8_t)err_sh);
 }
 
 // ---- heuristic kernel (space.py:162-227) ---------------------------------------------------------------------
@@ -1397,7 +1418,7 @@ __global__ void __launch_bounds__(32 * EPC) irbpp_candidates_kernel(const Params
         if (Ktot < sel) zero_rows(Ktot);
     }
     if (lane == 0) {
-        if (dev_err) { P.r_error[renv] = (uint8_t)dev_err; if (P.h_error) P.h_error[renv] = (uint8_t)dev_err; }
+        if (dev_err) store_error(P, renv, (uint8_t)dev_err);
         if (P.dbg_nhull) P.dbg_nhull[env] = Ktot;
     }
     if (warp == 0) trace(6);

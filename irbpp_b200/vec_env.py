@@ -110,8 +110,7 @@ class LazyInfos(Sequence):
     when indexed (at N = 4096 eagerly building them would dominate the step).  Holds this step's private
     copy of the library's result block; the typed views are cut out of it on first use."""
 
-    _FIELDS = (("valid", np.bool_), ("counter", np.int32), ("ratio", np.float64),
-               ("ep_reward", np.float64), ("ep_len", np.int32))
+    _FIELDS = ("valid", "counter", "ratio", "ep_reward", "ep_len")
 
     def __init__(self, n, block, offsets, done, t_rel, borrowed=False):
         self._n, self._block, self._offsets, self._done, self._t = n, block, offsets, done, t_rel
@@ -129,7 +128,8 @@ class LazyInfos(Sequence):
     def _views(self):
         if self._v is None:
             n, b, o = self._n, self._block, self._offsets
-            self._v = {k: b[o[k]:o[k] + n * np.dtype(dt).itemsize].view(dt) for k, dt in self._FIELDS}
+            self._v = {k: b[o[k]:o[k] + n * dt.itemsize].view(np.bool_ if k == "valid" else dt)
+                       for k, dt in _lib.RESULT_FIELDS if k in self._FIELDS}
         return self._v
 
     def __len__(self):
@@ -350,22 +350,20 @@ class GpuVecEnv(VecEnv):
             if old is not None:
                 old.detach()
 
-    _RESULT_BYTES = (("ratio", 8), ("ep_reward", 8), ("reward", 4), ("counter", 4), ("ep_len", 4),
-                     ("done", 1), ("valid", 1), ("error", 1))
-
     def _result_block(self, res):
-        """uint8 view of the library's pinned result block and the byte offset of every array in it (from
-        the pointers of ``irbpp_step_result``; two blocks per handle, each view built once)."""
-        key = (res.reward, res.done)
+        """uint8 view of the library's pinned result block that the pointers of ``irbpp_step_result`` point into,
+        and the byte offset of every array in it (two blocks per handle, each view built once).  Raises when a
+        pointer is not where ``_lib.RESULT_FIELDS`` puts it."""
+        base = getattr(res, _lib.RESULT_FIELDS[0][0])
         cache = self.__dict__.setdefault("_block_cache", {})      # the library alternates between two blocks
-        hit = cache.get(key)
+        hit = cache.get(base)
         if hit is None:
-            n = self.num_envs
-            ptrs = {k: getattr(res, k) for k, _ in self._RESULT_BYTES}
-            base = min(ptrs.values())
-            end = max(ptrs[k] + n * sz for k, sz in self._RESULT_BYTES)
-            buf = (ctypes.c_uint8 * (end - base)).from_address(base)
-            hit = cache[key] = (np.frombuffer(buf, dtype=np.uint8), {k: ptrs[k] - base for k, _ in self._RESULT_BYTES})
+            offsets, size = _lib.result_offsets(self.num_envs)
+            for k, off in offsets.items():
+                if getattr(res, k) != base + off:
+                    raise RuntimeError("result block: %s at byte %d, expected %d" % (k, getattr(res, k) - base, off))
+            buf = (ctypes.c_uint8 * size).from_address(base)
+            hit = cache[base] = (np.frombuffer(buf, dtype=np.uint8), offsets)
         return hit
 
     def step_device(self, actions):
@@ -396,9 +394,8 @@ class GpuVecEnv(VecEnv):
             class _View(object):
                 def __init__(self, ptr, shape, typestr):
                     self.__cuda_array_interface__ = {"shape": shape, "typestr": typestr, "data": (int(ptr), False), "version": 2}
-            spec = {"reward": "<f4", "done": "|u1", "valid": "|u1", "counter": "<i4", "ratio": "<f8", "ep_len": "<i4", "ep_reward": "<f8"}
-            views = self._dev_views = {k: torch.as_tensor(_View(getattr(res, k), (n,), ts), device=self.device)
-                                       for k, ts in spec.items()}
+            views = self._dev_views = {k: torch.as_tensor(_View(getattr(res, k), (n,), dt.str), device=self.device)
+                                       for k, dt in _lib.RESULT_FIELDS if k != "error"}
         return views
 
     def get_action_candidates(self, order_actions, as_tensor=False):

@@ -13,6 +13,7 @@ import numpy as np
 import pytest
 
 from conftest import lib_from_fixture, load_golden
+from irbpp_b200 import _lib
 
 pytestmark = pytest.mark.timeout(900)          # a deadlocked emulated barrier must not hang the suite
 
@@ -62,24 +63,13 @@ def emu(tmp_path_factory):
     return build_emulated(str(tmp_path_factory.mktemp("emu")))
 
 
-class _Cfg(ctypes.Structure):
-    _fields_ = [("num_envs", ctypes.c_int32), ("num_rotations", ctypes.c_int32), ("selected_action", ctypes.c_int32),
-                ("buffer_size", ctypes.c_int32), ("bin_dimension", ctypes.c_double * 3), ("resolution_act", ctypes.c_double),
-                ("resolution_h", ctypes.c_double), ("resolution_z", ctypes.c_double), ("device", ctypes.c_int32),
-                ("approx_legacy", ctypes.c_int32)]
-
-
-class _Res(ctypes.Structure):
-    _fields_ = [(n, ctypes.c_void_p) for n in ("reward", "done", "valid", "error", "counter", "ep_len", "ratio", "ep_reward")]
-
-
 class EmuEnv(object):
     """The C ABI of include/irbpp.h driven with NumPy buffers (device == host under the emulation)."""
 
     def __init__(self, lib, library, sequences, selected_action=500, buffer_size=1):
         self.lib, self.n = lib, len(sequences)
-        cfg = _Cfg(self.n, library.num_rotations, selected_action, buffer_size, (ctypes.c_double * 3)(0.32, 0.32, 0.30),
-                   0.02, 0.01, 0.01, 0, 0)
+        cfg = _lib.IrbppConfig(self.n, library.num_rotations, selected_action, buffer_size,
+                               (ctypes.c_double * 3)(0.32, 0.32, 0.30), 0.02, 0.01, 0.01, 0, 0)
         self.h = ctypes.c_void_p()
         assert lib.emu_irbpp_create(ctypes.byref(cfg), ctypes.byref(self.h)) == 0
         dims, ext, vol, maps, offsets = library.flat()
@@ -102,7 +92,7 @@ class EmuEnv(object):
         acts = np.ascontiguousarray(actions, dtype=np.int64)
         obs = np.zeros((self.n, self.obs_len), np.float32)
         assert self.lib.emu_irbpp_step_async(self.h, ctypes.c_void_p(acts.ctypes.data), 0, ctypes.c_void_p(obs.ctypes.data), None) == 0
-        res = _Res()
+        res = self.result = _lib.IrbppStepResult()
         assert self.lib.emu_irbpp_step_wait(self.h, ctypes.byref(res)) == 0, self.lib.emu_irbpp_last_error(self.h)
         view = lambda p, ct, dt: np.frombuffer((ct * self.n).from_address(p), dtype=dt).copy()
         return (obs, view(res.reward, ctypes.c_float, np.float32), view(res.done, ctypes.c_uint8, np.bool_),
@@ -145,6 +135,20 @@ def _replay(lib, name, steps):
                                         ("episode_truncate", 6), ("episode_buffered", 6), ("episode_buffered10", 5), ("episode_rot24", 3)])
 def test_emulated_kernels_replay_reference_episodes(emu, name, steps):
     _replay(emu, name, steps)
+
+
+def test_emulated_result_block_layout_matches_python_table(emu):
+    """The pointers irbpp_step_wait returns sit at the offsets of _lib.RESULT_FIELDS in a block of 31 bytes per bin."""
+    from irbpp_b200 import shapes
+    n = 5
+    lib = shapes.make_blockout_library(8, seed=1)
+    env = EmuEnv(emu, lib, shapes.make_sequences(n, 8, lib.num_shapes, seed=0))
+    env.reset()
+    env.step(np.zeros(n, np.int64))
+    offsets, size = _lib.result_offsets(n)
+    res = env.result
+    assert {k: getattr(res, k) - res.ratio for k in offsets} == offsets and size == 31 * n
+    env.close()
 
 
 
